@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
                     [--algo PPOLag|CPO|TRPOLag|FOCOPS] [--obs-dim D] [--precision bf16x3|tf32|fp32]
+                    [--dump-outputs DIR]
 
 A "step" is one epoch of a BASELINE.json workload: by default `configs[1]` = PPOLag on the synthetic Box env
 (obs 60 / act 8), 4096 HBM-resident envs per GPU, T = 128 steps per env (524 288 samples per GPU), update_iters 8,
@@ -17,6 +18,11 @@ batch_size 16384 -- i.e. the reference's `Time/FPS = steps_per_epoch / epoch_tim
   e2e     : the same metric through the public `omnisafe_b200.Agent(...)` training loop with HOST buffers: every
             epoch the standard-normal action-noise stream is copied from pinned host memory (parity-mode input of
             the rollout) and the epoch's logged metrics are read back.
+  --dump-outputs DIR : after the timed steps, what the last timed epoch handed its caller is written as DIR/<name>.npy
+            (float32; float64 where the library keeps float64): the parameters after the update, the epoch's rollout and
+            GAE slabs (a fixed, seeded sample of their (t, env) rows), the observation-normaliser statistics, the
+            episode-window sums, the update statistics and the Lagrange state.  The workload is seeded, so the same
+            arguments give the same inputs from run to run and two builds can be compared output for output.
   --impl reference : the CPU restatement of the reference path (oracle/, torch-CPU + numpy) timed on the host cores
             on the SAME workload size (4096 envs x T = 128 per step); /root/reference does not exist on the GPU box.
 """
@@ -135,6 +141,30 @@ def _flops_per_sample(O: int, A: int) -> int:
     return net(A) + 2 * net(1)
 
 
+DUMP_ROWS = 16384          # (t, env) rows of each per-epoch slab written by --dump-outputs: 5 MB at obs_dim 60
+
+
+def dump_outputs(algo, out_dir: str) -> None:
+    """--dump-outputs: the outputs of the epoch algo.train_epoch() last ran, as DIR/<name>.npy."""
+    d, env = algo._buf.data, algo._env
+    T, N = d['reward'].shape
+    rows = np.sort(np.random.default_rng(0).choice(T * N, size=min(DUMP_ROWS, T * N), replace=False))
+    rows = torch.as_tensor(rows, device=d['reward'].device)
+    out = {'theta': algo._actor_critic.theta, 'obs_norm_mean': env._obs_normalizer.mean,
+           'obs_norm_std': env._obs_normalizer.std, 'window_sums': env.window_sums,
+           'train_stats': algo._engine.train_stats, 'kl_state': algo._engine.kl_state, 'sample_rows': rows}
+    lagrange = getattr(algo, '_lagrange', None)
+    if lagrange is not None:
+        out['lagrange_state'] = lagrange.state
+    for name, v in d.items():
+        if v is not None and tuple(v.shape[:2]) == (T, N):
+            out['slab_' + name] = v.reshape(T * N, *v.shape[2:])[rows]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        v = v.detach().cpu()
+        np.save(os.path.join(out_dir, name + '.npy'), v.numpy().astype(np.float64 if v.dtype in (torch.float64, torch.int64) else np.float32))
+
+
 def run_b200(args) -> dict:
     import torch.distributed as dist
 
@@ -191,6 +221,8 @@ def run_b200(args) -> dict:
         ms = timed(algo.train_epoch, args.steps)
     launches = int(lib().osb_launch_count() - l0)
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(algo, args.dump_outputs)
     ms_per_step = ms / args.steps
     value = samples_global / (ms_per_step * 1e-3)
 
@@ -446,7 +478,12 @@ def main() -> None:
     ap.add_argument('--precision', default='bf16x3', choices=['bf16x3', 'tf32', 'fp32'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-extras', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the b200 path (--impl b200)')
     # stdout carries exactly ONE JSON line: whatever libraries print while the bench runs (e.g. NCCL's version banner, written
     # by C code straight to fd 1) is sent to stderr
     sys.stdout.flush()

@@ -1,14 +1,12 @@
-"""CPU, build container only: every shipped YAML `defaults` block equals the upstream block of the same
-algorithm key for key (plus the `matmul_precision` extension and the env_cfgs placeholder).  Skipped where
-/root/reference does not exist (GPU box)."""
+"""CPU: every shipped YAML `defaults` block equals the upstream block of the same algorithm key for key (plus the
+`matmul_precision` extension and the env_cfgs placeholder).  The upstream blocks are recorded from the unmodified
+reference in tests/golden/reference_configs.json (tests/golden/make_golden_reference_api.py)."""
+import json
 import os
 
-import pytest
 import yaml
 
-REF = '/root/reference/omnisafe/configs/on-policy'
 MINE = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), 'omnisafe_b200', 'configs', 'on-policy')
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason='reference tree not present')
 
 
 def _flat(d, pre=''):
@@ -21,14 +19,16 @@ def _flat(d, pre=''):
     return out
 
 
-def test_yaml_defaults_equal_upstream():
+def test_yaml_defaults_equal_upstream(golden_dir):
     from omnisafe_b200.algorithms import ALGORITHMS
 
+    with open(os.path.join(golden_dir, 'reference_configs.json')) as fh:
+        upstream = json.load(fh)
     names = sorted(f[:-5] for f in os.listdir(MINE) if f.endswith('.yaml'))
     assert set(names) == set(ALGORITHMS['on-policy'])          # one YAML per registered class
+    assert set(names) == set(upstream)                          # and one recorded upstream block per YAML
     for name in names:
-        with open(os.path.join(REF, name + '.yaml')) as fh:
-            ref = _flat(yaml.safe_load(fh)['defaults'])
+        ref = upstream[name]
         with open(os.path.join(MINE, name + '.yaml')) as fh:
             doc = yaml.safe_load(fh)
         mine = _flat(doc['defaults'])
