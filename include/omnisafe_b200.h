@@ -296,8 +296,9 @@ int osb_pid_lagrange_update(const double* window_sums, double pid_kp, double pid
                             int pid_d_delay, double pid_delta_p_ema_alpha, double pid_delta_d_ema_alpha,
                             int sum_norm, int diff_norm, double penalty_max, double cost_limit,
                             double* pid_state, float* lagrange_state, int* nan_flag, void* stream);
-/* kl = eval_out[0]/eval_out[4]; kl_state[4] = {last kl, passes done, stopped, 0}. */
-int osb_kl_check(const double* eval_out, float target_kl, int early_stop, int* stop_flag,
+/* kl = (float)(eval_out[0]/eval_out[4]); stops when (double)kl > target_kl, the reference's fp32 `kl.item() > target_kl`;
+ * kl_state[4] = {last kl, passes done, stopped, 0}. */
+int osb_kl_check(const double* eval_out, double target_kl, int early_stop, int* stop_flag,
                  float* kl_state, void* stream);
 /* out[q] = scale * sum_b gpart[b*stride + q] + add_scale * add[q], q < n  (add may be NULL). */
 int osb_reduce_partials(const float* gpart, int nblocks, int stride, int n, float scale,
@@ -325,7 +326,7 @@ int osb_ppo_update_epoch(float* theta, float* grad, float* adam_m, float* adam_v
                          int update_iters, int loss_kind, float clip, float entropy_coef,
                          float focops_lam, float focops_eta, const float* lagrange, int net_mask,
                          float critic_norm_coef, float max_grad_norm, float lr_actor,
-                         float lr_critic, float target_kl, int kl_early_stop, float* gpart,
+                         float lr_critic, double target_kl, int kl_early_stop, float* gpart,
                          float* stats_part, float* sumsq_part, float* train_stats, double* eval_ws,
                          double* eval_out, int* stop_flag, float* kl_state, int precision,
                          void* comm, int world_size, void* peer_buf, void* peer_flag, int rank,

@@ -78,7 +78,7 @@ int osb_optim_fused_p2p(const float* gpart, const float* stats_part, int nblocks
                         float lr_critic_r, float lr_critic_c, int net_mask, float* sumsq_part,
                         float* train_stats, const int* stop_flag, void* peer_buf, void* peer_flag,
                         int world, int rank, unsigned step_id, int* error_flag, void* stream);
-int osb_kl_check(const double* eval_out, float target_kl, int early_stop, int* stop_flag,
+int osb_kl_check(const double* eval_out, double target_kl, int early_stop, int* stop_flag,
                  float* kl_state, void* stream);
 }
 
@@ -178,7 +178,7 @@ int osb_ppo_update_epoch(float* theta, float* grad, float* adam_m, float* adam_v
                          int update_iters, int loss_kind, float clip, float entropy_coef,
                          float focops_lam, float focops_eta, const float* lagrange, int net_mask,
                          float critic_norm_coef, float max_grad_norm, float lr_actor,
-                         float lr_critic, float target_kl, int kl_early_stop, float* gpart,
+                         float lr_critic, double target_kl, int kl_early_stop, float* gpart,
                          float* stats_part, float* sumsq_part, float* train_stats, double* eval_ws,
                          double* eval_out, int* stop_flag, float* kl_state, int precision,
                          void* comm, int world_size, void* peer_buf, void* peer_flag, int rank,

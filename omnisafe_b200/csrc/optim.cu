@@ -388,15 +388,17 @@ __global__ void pid_lagrange_kernel(const double* __restrict__ window_sums, doub
 }
 
 // KL early stop: eval_out[0] = sum KL (over samples and action dims), eval_out[4] = sample count.
-// kl_state[4] = {last kl, iterations executed, stopped flag as float, 0}
-__global__ void kl_check_kernel(const double* __restrict__ eval_out, float target_kl, int early_stop,
+// kl_state[4] = {last kl, iterations executed, stopped flag as float, 0}.  The reference compares the fp32 KL with a Python
+// float (`kl.item() > target_kl`, policy_gradient.py:L395), so the test is done in double against the double target: a
+// float target would round e.g. 0.1 up to 0.100000001 and miss a KL of exactly that float.
+__global__ void kl_check_kernel(const double* __restrict__ eval_out, double target_kl, int early_stop,
                                 int* __restrict__ stop_flag, float* __restrict__ kl_state) {
     if (threadIdx.x != 0) return;
     if (*stop_flag) return;
     const float kl = (float)(eval_out[0] / eval_out[4]);
     kl_state[0] = kl;
     kl_state[1] += 1.f;
-    if (early_stop && kl > target_kl) { *stop_flag = 1; kl_state[2] = 1.f; }
+    if (early_stop && (double)kl > target_kl) { *stop_flag = 1; kl_state[2] = 1.f; }
 }
 
 // out[q] = scale * sum_b gpart[b][q] + add_scale * add[q]
@@ -620,7 +622,7 @@ int osb_pid_lagrange_update(const double* window_sums, double pid_kp, double pid
     return OSB_OK;
 }
 
-int osb_kl_check(const double* eval_out, float target_kl, int early_stop, int* stop_flag,
+int osb_kl_check(const double* eval_out, double target_kl, int early_stop, int* stop_flag,
                  float* kl_state, void* stream) {
     OSB_CHECK_ARG(eval_out && stop_flag && kl_state, "null pointer");
     kl_check_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(eval_out, target_kl, early_stop, stop_flag, kl_state);
