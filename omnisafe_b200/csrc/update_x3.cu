@@ -6,9 +6,13 @@
 // omnisafe/utils/model.py:L105-111).
 //
 // One CTA = one network x a strided set of 128-sample tiles (same grid / per-CTA partial-gradient contract as
-// minibatch_grad_tc_kernel).  Warp-specialised: 16 epilogue warps + 1 MMA-issue warp, linked by mbarriers only:
+// minibatch_grad_tc_kernel).  Warp-specialised: 16 epilogue warps + 1 MMA-issue warp, linked by mbarriers only.
+// Each 128-sample tile is worked as two 64-sample halves a / b, each with its own activation buffers, TMEM
+// columns, mbarriers and group of 8 epilogue warps; the MMA warp issues every stage for a, then b, so the tensor
+// core runs one half's GEMM while the other half's epilogue works (chain GEMMs at M = 64, weight-gradient GEMMs
+// with K = 64 samples per half into accumulators shared by both halves):
 //
-//   per tile (activations stored ONCE as [sample][feature] bf16x3 tiles; the weight-gradient GEMMs read the
+//   per half tile (activations stored ONCE as [sample][feature] bf16x3 tiles; the weight-gradient GEMMs read the
 //   same tiles MN-major, so there are no transposed copies):
 //     Z1   = X  W1^T            -> H1 = tanh(. + b1)
 //     Z2   = H1 W2^T            -> H2 = tanh(. + b2)
@@ -36,7 +40,7 @@ namespace osb {
 using namespace x3;
 
 __device__ __forceinline__ void epi_bar_sync() { asm volatile("bar.sync 1, 512;\n" ::: "memory"); }      // epilogue warps only
-__device__ __forceinline__ void loss_bar_sync() { asm volatile("bar.sync 2, 128;\n" ::: "memory"); }     // loss warps (h == 0)
+__device__ __forceinline__ void half_bar_sync(int hf) { asm volatile("bar.sync %0, 256;\n" ::"r"(2 + hf) : "memory"); }   // epilogue warps of half hf
 
 enum X3Loss { X3_PPO_CLIP = 0, X3_RATIO = 1, X3_FOCOPS = 2, X3_COST = 3, X3_FVP = 4, X3_P3O = 5 };   // X3_FVP: dOUT supplied (Fisher-vector product)
 
@@ -79,30 +83,40 @@ struct X3Args {
     long long* dbg;              // optional clock64 stamps of CTA (0, 0): [0] = count, then (id, clock) pairs (tools/x3_stage_times.py)
 };
 
-constexpr int XT = 128;                      // samples per tile
-constexpr int NEPI = 512;                    // 16 epilogue warps: lane quarter q = warp % 4, column group h = warp / 4
+constexpr int XT = 128;                      // samples per tile (the unit the tiles are dealt to the CTAs in)
+constexpr int HT = 64;                       // samples per half tile: the halves a / b of a tile alternate between the tensor
+                                             // core and their epilogue group, so GEMMs of one half run under the epilogue of the other
+constexpr int NEPI = 512;                    // 16 epilogue warps: half hf = warp / 8, lane quarter q = warp % 4
+constexpr int NGRP = NEPI / 2;               // epilogue threads of one half
 constexpr int NTX3 = NEPI + 32;              // + the MMA-issue warp
-constexpr uint32_t ACT_SUB = XT * 128, ACT_X3 = 3 * ACT_SUB;        // [128][64] bf16 sub-tile, x3 tile
-constexpr uint32_t D_SUB = XT * 32, D_X3 = 3 * D_SUB;               // [128][16] bf16 (SW32)
+constexpr uint32_t ACT_SUB = HT * 128, ACT_X3 = 3 * ACT_SUB;        // [64][64] bf16 sub-tile, x3 half tile
+constexpr uint32_t D_SUB = HT * 32, D_X3 = 3 * D_SUB;               // [64][16] bf16 (SW32)
 constexpr uint32_t W_SUB = 64 * 128, W_X3 = 3 * W_SUB;              // [64][64]
 constexpr uint32_t W3_SUB = 16 * 128, W3_X3 = 3 * W3_SUB;           // [16][64]
 constexpr uint32_t W_IMG = 2 * W_X3 + W3_X3;                         // 55 296 B: the weight tiles W1 | W2 | W3 as they sit in shared memory
-constexpr uint32_t OFF_X = 0, OFF_H1 = OFF_X + ACT_X3, OFF_H2 = OFF_H1 + ACT_X3, OFF_D = OFF_H2 + ACT_X3,
-                   OFF_W1 = OFF_D + D_X3, OFF_W2 = OFF_W1 + W_X3, OFF_W3 = OFF_W2 + W_X3, OFF_ONES = OFF_W3 + W3_X3,
+// activation buffers: half a, then half b (half hf of X at OFF_X + hf * ACT_X3, of D at OFF_D + hf * D_X3)
+constexpr uint32_t OFF_X = 0, OFF_H1 = OFF_X + 2 * ACT_X3, OFF_H2 = OFF_H1 + 2 * ACT_X3, OFF_D = OFF_H2 + 2 * ACT_X3,
+                   OFF_W1 = OFF_D + 2 * D_X3, OFF_W2 = OFF_W1 + W_X3, OFF_W3 = OFF_W2 + W_X3, OFF_ONES = OFF_W3 + W3_X3,
                    OFF_MISC = OFF_ONES + 512;
 // misc region (floats unless noted)
 constexpr int MF_B1 = 0, MF_B2 = 64, MF_B3 = 128, MF_LS = 144 /* logstd[16] sigma[16] dlogstd acc[16] */, MF_STAT = 192,
               MF_RED = 200 /* [4*8 + 4*16 + 4*16] */, MF_B3ACC = 360, MF_PART = 376 /* [2][256] */, MF_SCAL = 888 /* [16] */, MF_OLD = 904 /* log sigma_old[16], 1 / sigma_old^2 [16] */, MF_END = 936;
 constexpr uint32_t OFF_ROWS = OFF_MISC + MF_END * 4;                 // long long [2][128]
 constexpr uint32_t OFF_BARS = OFF_ROWS + 2 * XT * 8;                 // uint64 [NBAR]
-enum Bar { RDY_X0 = 0, RDY_X1, RDY_H1_0, RDY_H1_1, RDY_H2_0, RDY_H2_1, RDY_D, RDY_DZ2_0, RDY_DZ2_1, RDY_DZ1,
-           DONE_C1, DONE_C2, DONE_C3, DONE_C4A, DONE_C4B, DONE_C5A, DONE_C5B, DONE_C6, RDY_W, NBAR };
+// mbarriers of one half (barrier b of half hf: index hf * NHB + b), then the weight-image barrier
+enum HalfBar { RDY_X0 = 0, RDY_X1, RDY_H1_0, RDY_H1_1, RDY_H2_0, RDY_H2_1, RDY_D, RDY_DZ2_0, RDY_DZ2_1, RDY_DZ1,
+               DONE_C1, DONE_C2, DONE_C3, DONE_C4A, DONE_C4B, DONE_C5A, DONE_C5B, DONE_C6, NHB };
+constexpr int RDY_W = 2 * NHB, NBAR = 2 * NHB + 1;
 constexpr uint32_t OFF_TMEMSLOT = OFF_BARS + NBAR * 8;
 constexpr uint32_t OFF_PF = OFF_TMEMSLOT + 16;                        // float [128][12]: per-sample loss inputs (AP == 8), copied asynchronously
 constexpr int PF_LD = 12;
 constexpr uint32_t X3_SMEM = OFF_PF + XT * PF_LD * 4;
-// TMEM columns
-constexpr uint32_t T_ZA = 0, T_ZB = 64, T_OUT = 128, T_DW1 = 144, T_DW2 = 208, T_DW3 = 272, T_DB1 = 288, T_DB2 = 304, T_COLS = 512;
+static_assert(XT * (5 + 2 * 16) * 4 <= 2 * ACT_X3, "per-row loss sums must fit the H2 buffers");
+static_assert(1024 + X3_SMEM <= 227 * 1024, "dynamic shared memory of the bf16x3 update kernel exceeds 227 KB");
+// TMEM columns: per half Z_A | Z_B | OUT (half hf at hf * T_HALF), then the weight / bias gradients shared by both halves
+constexpr uint32_t T_ZA = 0, T_ZB = 64, T_OUT = 128, T_HALF = 144;
+constexpr uint32_t T_DW1 = 2 * T_HALF, T_DW2 = T_DW1 + 64, T_DW3 = T_DW2 + 64, T_DB1 = T_DW3 + 16, T_DB2 = T_DB1 + 16, T_COLS = 512;
+static_assert(T_DB2 + 16 <= T_COLS, "TMEM columns");
 
 __device__ __forceinline__ unsigned long long x3_feistel(unsigned long long k, unsigned long long n, unsigned seed) {
     int bits = 2;
@@ -248,7 +262,8 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
     } else {
         if (lane == 0) {
             for (int i = 0; i < NBAR; ++i) {
-                const uint32_t cnt = (i >= DONE_C1) ? 1u : (i == RDY_D ? 4u : 16u);      // (RDY_W: one expect_tx arrival)
+                const int b = i % NHB;          // producers: the 8 warps of a half, its 4 loss warps, one commit / expect_tx (RDY_W)
+                const uint32_t cnt = (i == RDY_W || b >= DONE_C1) ? 1u : (b == RDY_D ? 4u : 8u);
                 asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;\n" ::"r"(bar(i)), "r"(cnt) : "memory");
             }
             mbar_init_fence();
@@ -268,8 +283,12 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
         const uint64_t dX = desc128(sbase + OFF_X), dH1 = desc128(sbase + OFF_H1), dH2 = desc128(sbase + OFF_H2);
         const uint64_t dD = desc32(sbase + OFF_D), dW1 = desc128(sbase + OFF_W1), dW2 = desc128(sbase + OFF_W2);
         const uint64_t dW3 = desc128(sbase + OFF_W3), dOnes = desc32(sbase + OFF_ONES);
-        const uint32_t id_fwd = idesc_bf16(128, 64, 0, 0), id_out = idesc_bf16(128, 16, 0, 0), id_bwd = idesc_bf16(128, 64, 0, 1);
+        // chain GEMMs: M = 64 samples of one half; weight-gradient GEMMs: M = 64 weight rows, K = the 64 samples of one half
+        const uint32_t id_fwd = idesc_bf16(64, 64, 0, 0), id_out = idesc_bf16(64, 16, 0, 0), id_bwd = idesc_bf16(64, 64, 0, 1);
         const uint32_t id_dw = idesc_bf16(64, 64, 1, 1), id_dw16 = idesc_bf16(64, 16, 1, 1);
+        const bool backward = !(!FUSED && p.forward_only);       // forward-only statistics pass (FOCOPS / P3O pass 1): no backward
+        auto hbar = [&](int hf, int b) { return bar(hf * NHB + b); };
+        auto commit = [&](int hf, int b) { if (leader) mma_commit_a(hbar(hf, b)); __syncwarp(); };
         int it = 0;
 #pragma unroll 1
         for (int mb = 0; mb < n_mb; ++mb) {
@@ -278,75 +297,101 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
 #pragma unroll 1
             for (int tile = blockIdx.x; tile < ntiles; tile += G, ++it) {
                 const uint32_t par = (uint32_t)(it & 1);
-                const bool first = tile == (int)blockIdx.x;         // the first tile of a minibatch overwrites the accumulators
+                const bool first = tile == (int)blockIdx.x;         // half a of the first tile of a minibatch overwrites the accumulators
                 const bool last = tile + G >= ntiles;
+                // Every stage is issued for half a, then half b: while the tensor core runs one half's GEMM, the
+                // epilogue group of the other half works on the previous result.
                 // Z1 = X W1^T  (k-steps 0-1 after the first column half of X, 2-3 after the second)
 #pragma unroll 1
-                for (int ph = 0; ph < 2; ++ph) {
-                    mbar_wait_a(bar(RDY_X0 + ph), par);
-                    tc_fence_after();
-                    gemm_x3_warp(leader, tmem + T_ZA, desc_add(dX, 64u * ph), ACT_SUB, 32u, desc_add(dW1, 64u * ph), W_SUB, 32u, id_fwd, 2, ph > 0);
+                for (int hf = 0; hf < 2; ++hf) {
+#pragma unroll 1
+                    for (int ph = 0; ph < 2; ++ph) {
+                        mbar_wait_a(hbar(hf, RDY_X0 + ph), par);
+                        tc_fence_after();
+                        gemm_x3_warp(leader, tmem + hf * T_HALF + T_ZA, desc_add(dX, hf * ACT_X3 + 64u * ph), ACT_SUB, 32u, desc_add(dW1, 64u * ph), W_SUB, 32u, id_fwd, 2, ph > 0);
+                    }
+                    commit(hf, DONE_C1);
                 }
-                if (leader) mma_commit_a(bar(DONE_C1));
-                __syncwarp();
-                // db2 of the PREVIOUS tile (dZ2 still sits in the H2 buffer until this tile's E2): runs under E1,
+                // db2 of the PREVIOUS tile (dZ2 still sits in the H2 buffers until this tile's E2): runs under E1,
                 // completes before Z2 (in-order pipe), so DONE_C2 covers it
-                if (!first && !(!FUSED && p.forward_only)) gemm_x3_warp(leader, tmem + T_DB2, dH2, ACT_SUB, 2048u, dOnes, 0u, 0u, id_dw16, 8, tile != (int)blockIdx.x + G);
+                if (!first && backward)
+#pragma unroll 1
+                    for (int hf = 0; hf < 2; ++hf)
+                        gemm_x3_warp(leader, tmem + T_DB2, desc_add(dH2, hf * ACT_X3), ACT_SUB, 2048u, dOnes, 0u, 0u, id_dw16, 4, hf > 0 || tile != (int)blockIdx.x + G);
                 // Z2 = H1 W2^T
 #pragma unroll 1
-                for (int ph = 0; ph < 2; ++ph) {
-                    mbar_wait_a(bar(RDY_H1_0 + ph), par);
-                    tc_fence_after();
-                    gemm_x3_warp(leader, tmem + T_ZB, desc_add(dH1, 64u * ph), ACT_SUB, 32u, desc_add(dW2, 64u * ph), W_SUB, 32u, id_fwd, 2, ph > 0);
+                for (int hf = 0; hf < 2; ++hf) {
+#pragma unroll 1
+                    for (int ph = 0; ph < 2; ++ph) {
+                        mbar_wait_a(hbar(hf, RDY_H1_0 + ph), par);
+                        tc_fence_after();
+                        gemm_x3_warp(leader, tmem + hf * T_HALF + T_ZB, desc_add(dH1, hf * ACT_X3 + 64u * ph), ACT_SUB, 32u, desc_add(dW2, 64u * ph), W_SUB, 32u, id_fwd, 2, ph > 0);
+                    }
+                    commit(hf, DONE_C2);
                 }
-                if (leader) mma_commit_a(bar(DONE_C2));
-                __syncwarp();
                 // OUT = H2 W3^T
 #pragma unroll 1
-                for (int ph = 0; ph < 2; ++ph) {
-                    mbar_wait_a(bar(RDY_H2_0 + ph), par);
-                    tc_fence_after();
-                    gemm_x3_warp(leader, tmem + T_OUT, desc_add(dH2, 64u * ph), ACT_SUB, 32u, desc_add(dW3, 64u * ph), W3_SUB, 32u, id_out, 2, ph > 0);
+                for (int hf = 0; hf < 2; ++hf) {
+#pragma unroll 1
+                    for (int ph = 0; ph < 2; ++ph) {
+                        mbar_wait_a(hbar(hf, RDY_H2_0 + ph), par);
+                        tc_fence_after();
+                        gemm_x3_warp(leader, tmem + hf * T_HALF + T_OUT, desc_add(dH2, hf * ACT_X3 + 64u * ph), ACT_SUB, 32u, desc_add(dW3, 64u * ph), W3_SUB, 32u, id_out, 2, ph > 0);
+                    }
+                    commit(hf, DONE_C3);
                 }
-                if (leader) mma_commit_a(bar(DONE_C3));
-                __syncwarp();
-                if (!FUSED && p.forward_only) continue;              // statistics pass (FOCOPS mask mean): no backward
+                if (!backward) continue;
                 // dZ2' = dOUT W3 ; dW3^T += H2^T dOUT
-                mbar_wait_a(bar(RDY_D), par);
-                tc_fence_after();
-                gemm_x3_warp(leader, tmem + T_ZA, dD, D_SUB, 32u, dW3, W3_SUB, 2048u, id_bwd, 1, false);
-                if (leader) mma_commit_a(bar(DONE_C4A));
-                __syncwarp();
-                gemm_x3_warp(leader, tmem + T_DW3, dH2, ACT_SUB, 2048u, dD, D_SUB, 512u, id_dw16, 8, !first);
-                if (leader) mma_commit_a(bar(DONE_C4B));
-                __syncwarp();
+#pragma unroll 1
+                for (int hf = 0; hf < 2; ++hf) {
+                    mbar_wait_a(hbar(hf, RDY_D), par);
+                    tc_fence_after();
+                    gemm_x3_warp(leader, tmem + hf * T_HALF + T_ZA, desc_add(dD, hf * D_X3), D_SUB, 32u, dW3, W3_SUB, 2048u, id_bwd, 1, false);
+                    commit(hf, DONE_C4A);
+                    gemm_x3_warp(leader, tmem + T_DW3, desc_add(dH2, hf * ACT_X3), ACT_SUB, 2048u, desc_add(dD, hf * D_X3), D_SUB, 512u, id_dw16, 4, !first || hf > 0);
+                    commit(hf, DONE_C4B);
+                }
                 // dZ1' = dZ2 W2 ; dW2 += dZ2^T H1
 #pragma unroll 1
-                for (int ph = 0; ph < 2; ++ph) {
-                    mbar_wait_a(bar(RDY_DZ2_0 + ph), par);
-                    tc_fence_after();
-                    gemm_x3_warp(leader, tmem + T_ZB, desc_add(dH2, 64u * ph), ACT_SUB, 32u, desc_add(dW2, 4096u * ph), W_SUB, 2048u, id_bwd, 2, ph > 0);
+                for (int hf = 0; hf < 2; ++hf) {
+#pragma unroll 1
+                    for (int ph = 0; ph < 2; ++ph) {
+                        mbar_wait_a(hbar(hf, RDY_DZ2_0 + ph), par);
+                        tc_fence_after();
+                        gemm_x3_warp(leader, tmem + hf * T_HALF + T_ZB, desc_add(dH2, hf * ACT_X3 + 64u * ph), ACT_SUB, 32u, desc_add(dW2, 4096u * ph), W_SUB, 2048u, id_bwd, 2, ph > 0);
+                    }
+                    commit(hf, DONE_C5A);
+                    gemm_x3_warp(leader, tmem + T_DW2, desc_add(dH2, hf * ACT_X3), ACT_SUB, 2048u, desc_add(dH1, hf * ACT_X3), ACT_SUB, 2048u, id_dw, 4, !first || hf > 0);
+                    commit(hf, DONE_C5B);
                 }
-                if (leader) mma_commit_a(bar(DONE_C5A));
-                __syncwarp();
-                gemm_x3_warp(leader, tmem + T_DW2, dH2, ACT_SUB, 2048u, dH1, ACT_SUB, 2048u, id_dw, 8, !first);
-                if (leader) mma_commit_a(bar(DONE_C5B));
-                __syncwarp();
                 // dW1 += dZ1^T X (column 63 = db1 with the ones column) ; last tile of the minibatch: its own db2
-                mbar_wait_a(bar(RDY_DZ1), par);
-                tc_fence_after();
-                gemm_x3_warp(leader, tmem + T_DW1, dH1, ACT_SUB, 2048u, dX, ACT_SUB, 2048u, id_dw, 8, !first);
-                if (!ones_col) gemm_x3_warp(leader, tmem + T_DB1, dH1, ACT_SUB, 2048u, dOnes, 0u, 0u, id_dw16, 8, !first);
-                if (last) gemm_x3_warp(leader, tmem + T_DB2, dH2, ACT_SUB, 2048u, dOnes, 0u, 0u, id_dw16, 8, !first);
-                if (leader) mma_commit_a(bar(DONE_C6));
-                __syncwarp();
+#pragma unroll 1
+                for (int hf = 0; hf < 2; ++hf) {
+                    mbar_wait_a(hbar(hf, RDY_DZ1), par);
+                    tc_fence_after();
+                    const bool acc = !first || hf > 0;
+                    gemm_x3_warp(leader, tmem + T_DW1, desc_add(dH1, hf * ACT_X3), ACT_SUB, 2048u, desc_add(dX, hf * ACT_X3), ACT_SUB, 2048u, id_dw, 4, acc);
+                    if (!ones_col) gemm_x3_warp(leader, tmem + T_DB1, desc_add(dH1, hf * ACT_X3), ACT_SUB, 2048u, dOnes, 0u, 0u, id_dw16, 4, acc);
+                    if (last) gemm_x3_warp(leader, tmem + T_DB2, desc_add(dH2, hf * ACT_X3), ACT_SUB, 2048u, dOnes, 0u, 0u, id_dw16, 4, acc);
+                    commit(hf, DONE_C6);
+                }
             }
         }
     } else {
         // ======================= epilogue warps ===============================================================
-        const int q = warp & 3, h = warp >> 2;
+        const int q = warp & 3, h = warp >> 2;          // lane quarter, column group of the gradient read-out
         const uint32_t lane_base = (uint32_t)(q * 32) << 16;
-        const int s_row = 32 * q + lane;                 // sample row of this thread in the [s][.] accumulators
+        // tile loop: the 8 warps of half hf = warp / 8 own its 64 samples; the M = 64 accumulators hold sample row
+        // 16 q + l in lane l < 16 of quarter q.  Warps with h2 == 0 (the loss warps) also run the loss, one lane l < 16 per sample.
+        const int hf = warp >> 3, h2 = h & 1, gtid = tid & (NGRP - 1);
+        const int s_row = 16 * q + (lane & 15);          // sample row of this thread in its half
+        const bool loss_warp = h2 == 0, loss_lane = loss_warp && lane < 16;
+        const uint32_t sX = sbase + OFF_X + hf * ACT_X3, sH1 = sbase + OFF_H1 + hf * ACT_X3, sH2 = sbase + OFF_H2 + hf * ACT_X3;
+        const uint32_t sD = sbase + OFF_D + hf * D_X3;
+        const uint32_t tHalf = tmem + lane_base + hf * T_HALF;
+        // column of this thread in column half ph: 32 ph + 16 h2 + 8 (lane / 16) .. + 7 (see tmem_ld8_m64)
+        const int ccol = 16 * h2 + 8 * (lane >> 4);
+        auto hbar = [&](int b) { return bar(hf * NHB + b); };
         const float lam = (p.lagrange != nullptr) ? __ldg(p.lagrange) : 0.f;
         float m_r = 0.f, s_r = 1.f, m_c = 0.f;
         if (p.b.moments) { m_r = __ldg(p.b.moments + 0); s_r = __ldg(p.b.moments + 1); m_c = __ldg(p.b.moments + 2); }
@@ -354,12 +399,12 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
         float* sB1 = misc + MF_B1; float* sB2 = misc + MF_B2; float* sB3 = misc + MF_B3; float* sLs = misc + MF_LS;
         float* sRed = misc + MF_RED; float* sPart = misc + MF_PART; float* sScal = misc + MF_SCAL;
 
-        // X gather: thread -> row xm = tid / 4, columns 32 ph + 8 (tid % 4) .. + 7 in column half ph
-        const int xm = tid >> 2, xc = (tid & 3) << 3;
+        // X gather: thread -> row xm = gtid / 4 of its half, columns 32 ph + 8 (gtid % 4) .. + 7 in column half ph
+        const int xm = gtid >> 2, xc = (gtid & 3) << 3;
         const bool vec = (O & 3) == 0;
         float xpre[16];
         auto prefetch_x = [&](const long long* rows) {
-            const long long row = rows[xm];
+            const long long row = rows[hf * HT + xm];
 #pragma unroll
             for (int ph = 0; ph < 2; ++ph) {
                 const int c0 = 32 * ph + xc;
@@ -382,7 +427,7 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
             fence_async_smem();
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) mbar_arrive(bar(b));
+            if (lane == 0) mbar_arrive(hbar(b));
         };
         const bool dbg_on = p.dbg != nullptr && blockIdx.x == 0 && blockIdx.y == 0 && (tid == 0 || tid == 256);
         int dbg_n = 0;
@@ -407,18 +452,18 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
             start = p.b.mb_start + (long long)mb * batch;
             count = min(batch, p.b.mb_count - mb * batch);
         };
-        auto tile_rows = [&](int mb, int tile, long long* dst) {
-            if (tid < XT) {
+        auto tile_rows = [&](int mb, int tile, long long* dst) {      // the loss lane of a sample writes its row
+            if (loss_lane) {
                 long long start; int count;
                 mb_geom(mb, start, count);
-                const int local = tile * XT + tid;
+                const int local = tile * XT + hf * HT + s_row;
                 long long row = -1;
                 if (local < count) {
                     const long long k = start + local;
                     if (p.b.identity_stride > 0) row = k * p.b.identity_stride;
                     else row = p.b.perm ? (long long)p.b.perm[k] : (long long)x3_feistel((unsigned long long)k, (unsigned long long)p.b.total, p.b.perm_seed);
                 }
-                dst[tid] = row;
+                dst[hf * HT + s_row] = row;
             }
         };
         int step_t0 = 0;
@@ -444,7 +489,7 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
         int rpar = 0, it = 0;
         if ((int)blockIdx.x < (min(batch, p.b.mb_count) + XT - 1) / XT) {     // rows + X of the first tile
             tile_rows(0, blockIdx.x, sRowBuf);
-            epi_bar_sync();
+            half_bar_sync(hf);
             prefetch_x(sRowBuf);
         }
 #pragma unroll 1
@@ -469,7 +514,7 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                 // ---- E0: X tile (prefetched registers -> bf16x3) ------------------------------------------------
                 stamp(0);
                 if (has_next) tile_rows(mb, tile + G, sRowNext);
-                if (it > 0 && !(!FUSED && p.forward_only)) mbar_wait_a(bar(DONE_C6), par ^ 1u);   // previous tile's dW1 / db1 read X and dZ1
+                if (it > 0 && !(!FUSED && p.forward_only)) mbar_wait_a(hbar(DONE_C6), par ^ 1u);   // previous tile's dW1 / db1 read X and dZ1
                 stamp(1);
                 tc_fence_after();
 #pragma unroll
@@ -477,23 +522,23 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                     float v[8];
 #pragma unroll
                     for (int i = 0; i < 8; ++i) v[i] = xpre[8 * ph + i];
-                    store8_x3(sbase + OFF_X, ACT_SUB, xm, 32 * ph + xc, v);
+                    store8_x3(sX, ACT_SUB, xm, 32 * ph + xc, v);
                     announce(RDY_X0 + ph);
                 }
-                epi_bar_sync();                                            // next tile's row list is complete
+                half_bar_sync(hf);                                         // next tile's row list is complete
                 stamp(2);
                 // loss warps: this tile's per-sample inputs (used in E3) fly under the forward phases -- asynchronously into
                 // shared memory when they fit (AP == 8), so that no register has to wait for them
                 float pf_act[AP], pf_logp = 0.f, pf_advr = 0.f, pf_advc = 0.f, pf_tv = 0.f;
                 long long prow = -1;
-                if (h == 0) {
-                    prow = sRow[s_row];
+                if (loss_warp) {
+                    if (loss_lane) prow = sRow[hf * HT + s_row];
 #pragma unroll
                     for (int a = 0; a < AP; ++a) pf_act[a] = 0.f;
                     if (prow >= 0) {
                         const float* asrc = (p.kind == X3_FVP) ? p.fvp_dmu : p.b.act;
                         if (AP == 8) {
-                            const uint32_t dst = sbase + OFF_PF + (uint32_t)(s_row * PF_LD) * 4u;
+                            const uint32_t dst = sbase + OFF_PF + (uint32_t)((hf * HT + s_row) * PF_LD) * 4u;
                             auto cp4 = [&](uint32_t d, const float* src) {
                                 asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(d), "l"(src) : "memory");
                             };
@@ -516,40 +561,40 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                     }
                 }
                 // ---- E1: H1 = tanh(Z1 + b1) -------------------------------------------------------------------
-                mbar_wait_a(bar(DONE_C1), par);
+                mbar_wait_a(hbar(DONE_C1), par);
                 tc_fence_after();
                 stamp(3);
 #pragma unroll
                 for (int ph = 0; ph < 2; ++ph) {
-                    const int c0 = 32 * ph + 8 * h;
+                    const int c0 = 32 * ph + ccol;
                     float v[8];
-                    tmem_ld8(tmem + lane_base + T_ZA + (uint32_t)c0, v);
+                    tmem_ld8_m64(tHalf + T_ZA + (uint32_t)(32 * ph + 16 * h2), v);
 #pragma unroll
                     for (int i = 0; i < 8; ++i) v[i] = tanh_acc(v[i] + sB1[c0 + i]);
-                    store8_x3(sbase + OFF_H1, ACT_SUB, s_row, c0, v);
+                    store8_x3(sH1, ACT_SUB, s_row, c0, v);
                     announce(RDY_H1_0 + ph);
                 }
                 // ---- E2: H2 = tanh(Z2 + b2) -------------------------------------------------------------------
                 stamp(4);
-                mbar_wait_a(bar(DONE_C2), par);
+                mbar_wait_a(hbar(DONE_C2), par);
                 tc_fence_after();
                 stamp(5);
 #pragma unroll
                 for (int ph = 0; ph < 2; ++ph) {
-                    const int c0 = 32 * ph + 8 * h;
+                    const int c0 = 32 * ph + ccol;
                     float v[8];
-                    tmem_ld8(tmem + lane_base + T_ZB + (uint32_t)c0, v);
+                    tmem_ld8_m64(tHalf + T_ZB + (uint32_t)(32 * ph + 16 * h2), v);
 #pragma unroll
                     for (int i = 0; i < 8; ++i) v[i] = tanh_acc(v[i] + sB2[c0 + i]);
-                    store8_x3(sbase + OFF_H2, ACT_SUB, s_row, c0, v);
+                    store8_x3(sH2, ACT_SUB, s_row, c0, v);
                     announce(RDY_H2_0 + ph);
                 }
                 stamp(6);
-                // ---- E3: OUT -> loss -> dOUT (warps with h == 0: one thread per sample) -------------------------
-                if (h == 0) {
+                // ---- E3: OUT -> loss -> dOUT (loss warps: one lane l < 16 per sample) --------------------------------
+                if (loss_warp) {
                     if (AP == 8) {
                         asm volatile("cp.async.wait_all;\n" ::: "memory");
-                        const float* pf = reinterpret_cast<const float*>(gbase + OFF_PF) + s_row * PF_LD;
+                        const float* pf = reinterpret_cast<const float*>(gbase + OFF_PF) + (hf * HT + s_row) * PF_LD;
                         if (prow >= 0) {
                             if (net == 0) {
 #pragma unroll
@@ -561,7 +606,7 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                             }
                         }
                     }
-                    mbar_wait_a(bar(DONE_C3), par);
+                    mbar_wait_a(hbar(DONE_C3), par);
                     tc_fence_after();
                     stamp(7);
                     float o[AP], d16[16];
@@ -569,12 +614,12 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                     for (int a = 0; a < 16; ++a) d16[a] = 0.f;
                     if (AP == 8) {
                         float t8[8];
-                        tmem_ld8(tmem + lane_base + T_OUT, t8);
+                        tmem_ld8(tHalf + T_OUT, t8);
 #pragma unroll
                         for (int a = 0; a < AP; ++a) o[a] = t8[a];
                     } else {
                         float t16[16];
-                        tmem_ld16(tmem + lane_base + T_OUT, t16);
+                        tmem_ld16(tHalf + T_OUT, t16);
 #pragma unroll
                         for (int a = 0; a < AP; ++a) o[a] = t16[a];
                     }
@@ -669,66 +714,66 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                                 }
                         }
                     }
-                    store16_x3_sw32(sbase + OFF_D, D_SUB, s_row, d16);
+                    if (lane < 16) store16_x3_sw32(sD, D_SUB, s_row, d16);
                     announce(RDY_D);
                     stamp(8);
                 }
                 stamp(9);
                 if (!FUSED && p.forward_only) {                                      // statistics pass: no backward; H2 is free once OUT is done
                     if (has_next) prefetch_x(sRowNext);
-                    if (h != 0) { mbar_wait_a(bar(DONE_C3), par); tc_fence_after(); }
+                    if (!loss_warp) { mbar_wait_a(hbar(DONE_C3), par); tc_fence_after(); }
                     rpar ^= 1;
                     continue;
                 }
                 // ---- E4: dZ2 = (dOUT W3) (1 - H2^2), stored over H2 once dW3 has read it --------------------------
                 if (has_next) prefetch_x(sRowNext);                        // next tile's rows fly during the backward half
-                mbar_wait_a(bar(DONE_C4A), par);
+                mbar_wait_a(hbar(DONE_C4A), par);
                 tc_fence_after();
                 stamp(10);
                 float dz[16];
 #pragma unroll
                 for (int ph = 0; ph < 2; ++ph) {
-                    const int c0 = 32 * ph + 8 * h;
+                    const int c0 = 32 * ph + ccol;
                     float v[8], hh[8];
-                    tmem_ld8(tmem + lane_base + T_ZA + (uint32_t)c0, v);
-                    load8_x3(sbase + OFF_H2, ACT_SUB, s_row, c0, hh);
+                    tmem_ld8_m64(tHalf + T_ZA + (uint32_t)(32 * ph + 16 * h2), v);
+                    load8_x3(sH2, ACT_SUB, s_row, c0, hh);
 #pragma unroll
                     for (int i = 0; i < 8; ++i) dz[8 * ph + i] = v[i] * (1.f - hh[i] * hh[i]);
                 }
                 stamp(11);
-                mbar_wait_a(bar(DONE_C4B), par);
+                mbar_wait_a(hbar(DONE_C4B), par);
                 stamp(12);
 #pragma unroll
                 for (int ph = 0; ph < 2; ++ph) {
                     float v[8];
 #pragma unroll
                     for (int i = 0; i < 8; ++i) v[i] = dz[8 * ph + i];
-                    store8_x3(sbase + OFF_H2, ACT_SUB, s_row, 32 * ph + 8 * h, v);
+                    store8_x3(sH2, ACT_SUB, s_row, 32 * ph + ccol, v);
                     announce(RDY_DZ2_0 + ph);
                 }
                 // ---- E5: dZ1 = (dZ2 W2) (1 - H1^2), stored over H1 once dW2 has read it --------------------------
                 stamp(13);
-                mbar_wait_a(bar(DONE_C5A), par);
+                mbar_wait_a(hbar(DONE_C5A), par);
                 tc_fence_after();
                 stamp(14);
 #pragma unroll
                 for (int ph = 0; ph < 2; ++ph) {
-                    const int c0 = 32 * ph + 8 * h;
+                    const int c0 = 32 * ph + ccol;
                     float v[8], hh[8];
-                    tmem_ld8(tmem + lane_base + T_ZB + (uint32_t)c0, v);
-                    load8_x3(sbase + OFF_H1, ACT_SUB, s_row, c0, hh);
+                    tmem_ld8_m64(tHalf + T_ZB + (uint32_t)(32 * ph + 16 * h2), v);
+                    load8_x3(sH1, ACT_SUB, s_row, c0, hh);
 #pragma unroll
                     for (int i = 0; i < 8; ++i) dz[8 * ph + i] = v[i] * (1.f - hh[i] * hh[i]);
                 }
                 stamp(15);
-                mbar_wait_a(bar(DONE_C5B), par);
+                mbar_wait_a(hbar(DONE_C5B), par);
                 stamp(16);
 #pragma unroll
                 for (int ph = 0; ph < 2; ++ph) {
                     float v[8];
 #pragma unroll
                     for (int i = 0; i < 8; ++i) v[i] = dz[8 * ph + i];
-                    store8_x3(sbase + OFF_H1, ACT_SUB, s_row, 32 * ph + 8 * h, v);
+                    store8_x3(sH1, ACT_SUB, s_row, 32 * ph + ccol, v);
                 }
                 announce(RDY_DZ1);
                 stamp(17);
@@ -741,40 +786,50 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                 mb_geom(mb + 1, s2, c2);
                 if ((int)blockIdx.x < (c2 + XT - 1) / XT) {
                     tile_rows(mb + 1, blockIdx.x, sRowBuf + rpar * XT);
-                    epi_bar_sync();
+                    half_bar_sync(hf);
                     prefetch_x(sRowBuf + rpar * XT);
                 }
             }
             // ---- this CTA's partial gradient of the minibatch: TMEM accumulators -> global ------------------------
             if (have_tiles) {
-                // loss-warp sums: lanes -> warp (butterfly) -> the four loss warps (fixed order)
-                if (h == 0) {
+                // Loss-lane partial sums, reduced exactly as with whole 128-sample tiles: each loss lane owns one tile row
+                // (hf * 64 + s_row) across the tiles; the rows go through shared memory (the H2 buffers, idle once the last MMA
+                // of the minibatch has completed) to threads 0-127, one row each, so warp q sums rows 32 q .. 32 q + 31
+                // (butterfly), then the four warps in a fixed order.
+                mbar_wait_a(bar(NHB + ((!FUSED && p.forward_only) ? DONE_C3 : DONE_C6)), (uint32_t)((it - 1) & 1));   // half b's last commit
+                tc_fence_after();
+                stamp(21);
+                constexpr int RLD = 5 + 2 * AP;
+                float* sLoss = reinterpret_cast<float*>(gbase + OFF_H2);
+                if (loss_lane) {
+                    float* r = sLoss + (hf * HT + s_row) * RLD;
 #pragma unroll
-                    for (int i = 0; i < 5; ++i) acc_st[i] = warp_sum(acc_st[i]);
+                    for (int i = 0; i < 5; ++i) { r[i] = acc_st[i]; acc_st[i] = 0.f; }
 #pragma unroll
-                    for (int a = 0; a < AP; ++a) { acc_dls[a] = warp_sum(acc_dls[a]); acc_db[a] = warp_sum(acc_db[a]); }
-                    if (lane == 0) {
+                    for (int a = 0; a < AP; ++a) { r[5 + a] = acc_dls[a]; r[5 + AP + a] = acc_db[a]; acc_dls[a] = 0.f; acc_db[a] = 0.f; }
+                }
+                epi_bar_sync();
+                if (tid < XT) {
+                    const float* r = sLoss + tid * RLD;
 #pragma unroll
-                        for (int i = 0; i < 5; ++i) sRed[q * 8 + i] = acc_st[i];
-#pragma unroll
-                        for (int a = 0; a < AP; ++a) { sRed[32 + q * 16 + a] = acc_dls[a]; sRed[96 + q * 16 + a] = acc_db[a]; }
+                    for (int i = 0; i < 5; ++i) {
+                        const float v = warp_sum(r[i]);
+                        if (lane == 0) sRed[q * 8 + i] = v;
                     }
 #pragma unroll
-                    for (int i = 0; i < 5; ++i) acc_st[i] = 0.f;
-#pragma unroll
-                    for (int a = 0; a < AP; ++a) { acc_dls[a] = 0.f; acc_db[a] = 0.f; }
+                    for (int a = 0; a < AP; ++a) {
+                        const float dl = warp_sum(r[5 + a]), db = warp_sum(r[5 + AP + a]);
+                        if (lane == 0) { sRed[32 + q * 16 + a] = dl; sRed[96 + q * 16 + a] = db; }
+                    }
                 }
                 if (!FUSED && p.forward_only) {
-                    epi_bar_sync();                    // sRed of the four loss warps
+                    epi_bar_sync();                    // sRed of the four reducing warps
                     if (tid >= 64 && tid < 72) {
                         const int i = tid - 64;
                         __stcg(p.stats_part + ((size_t)blockIdx.x * 3 + net) * 8 + i, (i < 5) ? (sRed[i] + sRed[8 + i]) + (sRed[16 + i] + sRed[24 + i]) : 0.f);
                     }
                     break;
                 }
-                mbar_wait_a(bar(DONE_C6), (uint32_t)((it - 1) & 1));
-                tc_fence_after();
-                stamp(21);
                 const int t_row = 16 * q + lane;       // row (lane < 16) of the M = 64 accumulators
                 const int c16 = 16 * h;
                 float v[16];
@@ -819,7 +874,7 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                     if (lane < 16) __stcg(gout + L.off_b2 + t_row, v[0]);
                 }
                 tc_fence_before();
-                epi_bar_sync();                        // sRed of the four loss warps
+                epi_bar_sync();                        // sRed of the four reducing warps
                 if (tid < L.out) __stcg(gout + L.off_b3 + tid, (sRed[96 + tid] + sRed[112 + tid]) + (sRed[128 + tid] + sRed[144 + tid]));
                 if (net == 0 && tid >= 32 && tid < 32 + A) {
                     const int a = tid - 32;

@@ -231,6 +231,18 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
 #pragma unroll
     for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
 }
+// M = 64 accumulator (row 16 q + l in lane l < 16 of lane quarter q): thread t < 16 receives row t, columns
+// [c, c + 8); thread t >= 16 row t - 16, columns [c + 8, c + 16) -- all 32 threads carry data.
+__device__ __forceinline__ void tmem_ld8_m64(uint32_t taddr, float (&v)[8]) {
+    uint32_t r[8];
+    asm volatile("tcgen05.ld.sync.aligned.16x32bx2.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8], 8;\n"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                 : "r"(taddr)
+                 : "memory");
+    asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory");
+#pragma unroll
+    for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
+}
 // 8 consecutive columns [c0, c0 + 8) (c0 % 8 == 0) of row r of a SW128 x3 tile
 __device__ __forceinline__ void store8_x3(uint32_t base, uint32_t split, int r, int c0, const float (&v)[8]) {
     uint32_t w0[4], w1[4], w2[4];

@@ -1,5 +1,7 @@
 """Where one CTA of the persistent bf16x3 update kernel spends its time: clock64 stamps of CTA (0, 0)
-(thread 0 = loss warp, thread 256 = a non-loss warp)."""
+(thread 0 = a loss warp of half tile a, thread 256 = a loss warp of half tile b; each half runs its own E0-E5 and
+waits on its own C* barriers).  One rank: stamp 26 only appears when clip_grad_norm_ clips (Adam redone + a third
+barrier), and stamp 27 follows the read of the clip coefficient."""
 import os, sys, tempfile
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -17,8 +19,8 @@ torch.cuda.synchronize()
 lib().osb_x3_debug_buffer(0)
 NAMES = {0: 'E0 start', 1: 'C6(prev) ok', 2: 'X stored+sync', 3: 'C1 ok', 4: 'E1 done', 5: 'C2 ok', 6: 'E2 done', 7: 'C3 ok', 8: 'dOUT stored', 9: 'E3 done',
          10: 'C4A ok', 11: 'E4 computed', 12: 'C4B ok', 13: 'E4 stored', 14: 'C5A ok', 15: 'E5 computed', 16: 'C5B ok', 17: 'E5 stored', 20: 'tiles done',
-         21: 'C6 ok', 22: 'extracted', 23: 'barrier1', 24: 'reduced', 25: 'barrier2', 26: 'adam done', 27: 'barrier3', 28: 'restaged'}
-for which, off in (('thread 0 (loss warp)', 0), ('thread 256', 1024)):
+         21: 'C6 ok', 22: 'extracted', 23: 'barrier1', 24: 'reduced', 25: 'barrier2', 26: 'clip redo+bar3', 27: 'clip coef read', 28: 'restaged'}
+for which, off in (('thread 0 (half a)', 0), ('thread 256 (half b)', 1024)):
     d = dbg[off:off + 1024].cpu().tolist()
     n = d[0]
     print(f'== {which}: {n} stamps (last update iteration kept the buffer)')
