@@ -11,6 +11,7 @@ import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
+INCLUDE = os.path.join(HERE, '..', 'include')
 LIBDIR = os.path.join(HERE, 'lib')
 LIB = os.path.join(LIBDIR, 'libomnisafe_b200.so')
 NVCC = os.environ.get('NVCC', '/usr/local/cuda/bin/nvcc')
@@ -28,11 +29,11 @@ def sources() -> list[str]:
 
 def _digest() -> str:
     h = hashlib.sha256()
-    for f in sorted(os.listdir(CSRC)):
-        if f.endswith(('.cu', '.cuh', '.h')):
-            with open(os.path.join(CSRC, f), 'rb') as fh:
-                h.update(f.encode())
-                h.update(fh.read())
+    files = [os.path.join(CSRC, f) for f in sorted(os.listdir(CSRC)) if f.endswith(('.cu', '.cuh', '.h'))]
+    for path in files + [os.path.join(INCLUDE, 'omnisafe_b200.h')]:   # every source includes the C-ABI header
+        with open(path, 'rb') as fh:
+            h.update(os.path.basename(path).encode())
+            h.update(fh.read())
     h.update(' '.join(FLAGS).encode())
     return h.hexdigest()
 
@@ -49,7 +50,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     procs = []
     for src in sources():
         obj = os.path.join(LIBDIR, os.path.basename(src)[:-3] + '.o')
-        cmd = [NVCC, *FLAGS, '-I', os.path.join(HERE, '..', 'include'), '-c', src, '-o', obj]
+        cmd = [NVCC, *FLAGS, '-I', INCLUDE, '-c', src, '-o', obj]
         if verbose:
             cmd.insert(1, '-Xptxas=-v')
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT)))

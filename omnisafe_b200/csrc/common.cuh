@@ -4,6 +4,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include "omnisafe_b200.h"   // the C ABI: every entry point is defined against its prototype here
+
 #define OSB_OK 0
 #define OSB_ERR_ARG 1
 #define OSB_ERR_CUDA 2

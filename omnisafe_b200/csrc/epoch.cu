@@ -7,81 +7,6 @@
 #include <stdlib.h>
 #include <string.h>
 
-extern "C" {
-int osb_update_grid_blocks(int mb_count);
-int osb_tc_grid_blocks(long long rows, int net_mask);
-int osb_minibatch_grad(const float* theta, int O, int A, const float* obs, const float* act,
-                       const float* logp, const float* adv_r, const float* adv_c,
-                       const float* tv_r, const float* tv_c, const float* mu_old,
-                       const float* moments, const int* perm, long long total, unsigned perm_seed,
-                       long long mb_start, int mb_count, int loss_kind, float clip,
-                       float entropy_coef, float focops_lam, float focops_eta,
-                       const float* lagrange, const float* logstd_old, int net_mask, float* gpart,
-                       float* stats_part, const int* stop_flag, void* stream);
-int osb_minibatch_grad_tc(const float* theta, int O, int A, const float* obs, const float* act,
-                          const float* logp, const float* adv_r, const float* adv_c,
-                          const float* tv_r, const float* tv_c, const float* mu_old,
-                          const float* moments, const int* perm, long long total, unsigned perm_seed,
-                          long long mb_start, int mb_count, int loss_kind, float clip,
-                          float entropy_coef, float focops_lam, float focops_eta,
-                          const float* lagrange, const float* logstd_old, int net_mask, float* gpart,
-                          float* stats_part, const int* stop_flag, void* stream);
-int osb_minibatch_grad_x3(const float* theta, int O, int A, const float* obs, const float* act,
-                          const float* logp, const float* adv_r, const float* adv_c,
-                          const float* tv_r, const float* tv_c, const float* mu_old,
-                          const float* moments, const int* perm, long long total, unsigned perm_seed,
-                          long long mb_start, int mb_count, int loss_kind, float clip,
-                          float entropy_coef, float focops_lam, float focops_eta,
-                          const float* lagrange, const float* logstd_old, int net_mask, float* gpart,
-                          float* stats_part, const int* stop_flag, void* stream);
-int osb_actor_eval(const float* theta_actor, int O, int A, const float* obs, const float* act,
-                   const float* logp, const float* adv_r, const float* adv_c, const float* mu_old,
-                   const float* logstd_old, const float* moments, const float* lagrange,
-                   long long total, int stride, float* mu_store, double* workspace, double* out,
-                   void* stream);
-int osb_actor_eval_tc(const float* theta_actor, int O, int A, const float* obs, const float* act,
-                      const float* logp, const float* adv_r, const float* adv_c, const float* mu_old,
-                      const float* logstd_old, const float* moments, const float* lagrange,
-                      long long total, int stride, float* mu_store, double* workspace, double* out,
-                      void* stream);
-int osb_ppo_update_iter_x3(float* theta, float* grad, float* adam_m, float* adam_v, int* adam_step, int O, int A,
-                           const float* obs, const float* act, const float* logp, const float* adv_r,
-                           const float* adv_c, const float* tv_r, const float* tv_c, const float* moments,
-                           const int* perm, long long total, unsigned perm_seed, int batch_size, int loss_kind,
-                           float clip, float entropy_coef, const float* lagrange, int net_mask,
-                           float critic_norm_coef, float max_grad_norm, float lr_actor, float lr_critic_r,
-                           float lr_critic_c, float* gpart, float* stats_part, float* train_stats,
-                           const int* stop_flag, void* peer_buf, void* peer_flag, int world, int rank,
-                           int* p2p_error, void* stream);
-int osb_actor_eval_x3(const float* theta_actor, int O, int A, const float* obs, const float* act,
-                      const float* logp, const float* adv_r, const float* adv_c, const float* mu_old,
-                      const float* logstd_old, const float* moments, const float* lagrange,
-                      long long total, int stride, float* mu_store, double* workspace, double* out,
-                      void* stream);
-int osb_grad_reduce(const float* gpart, const float* stats_part, int nblocks, int O, int A,
-                    const float* theta, float* grad, float critic_norm_coef, int net_mask,
-                    float* sumsq_part, int* adam_step, float* train_stats, const int* stop_flag,
-                    void* stream);
-int osb_clip_adam(float* grad, float* theta, float* adam_m, float* adam_v, const int* adam_step,
-                  const float* sumsq_part, int O, int A, float max_grad_norm, float lr_actor,
-                  float lr_critic_r, float lr_critic_c, float grad_scale, float critic_norm_coef,
-                  float* train_stats, int do_clip, int do_adam, int net_mask, const int* stop_flag,
-                  void* stream);
-int osb_optim_fused(const float* gpart, const float* stats_part, int nblocks, int O, int A,
-                    float* theta, float* grad, float* adam_m, float* adam_v, int* adam_step,
-                    float critic_norm_coef, float max_grad_norm, float lr_actor, float lr_critic_r,
-                    float lr_critic_c, int net_mask, float* sumsq_part, float* train_stats,
-                    const int* stop_flag, void* stream);
-int osb_optim_fused_p2p(const float* gpart, const float* stats_part, int nblocks, int O, int A,
-                        float* theta, float* grad, float* adam_m, float* adam_v, int* adam_step,
-                        float critic_norm_coef, float max_grad_norm, float lr_actor,
-                        float lr_critic_r, float lr_critic_c, int net_mask, float* sumsq_part,
-                        float* train_stats, const int* stop_flag, void* peer_buf, void* peer_flag,
-                        int world, int rank, unsigned step_id, int* error_flag, void* stream);
-int osb_kl_check(const double* eval_out, double target_kl, int early_stop, int* stop_flag,
-                 float* kl_state, void* stream);
-}
-
 // ---- NCCL through dlopen (the library torch already loaded; no link-time dependency) ----------
 namespace {
 typedef struct { char internal[128]; } nccl_uid_t;

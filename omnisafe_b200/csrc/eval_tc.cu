@@ -203,12 +203,6 @@ using namespace osb;
 
 extern "C" {
 
-// Tensor-core variant of osb_actor_eval (O <= 512; layer 1 K-chunked above 64); same arguments and outputs.
-int osb_actor_eval_tc(const float* theta_actor, int O, int A, const float* obs, const float* act,
-                      const float* logp, const float* adv_r, const float* adv_c, const float* mu_old,
-                      const float* logstd_old, const float* moments, const float* lagrange,
-                      long long total, int stride, float* mu_store, double* workspace, double* out,
-                      void* stream);
 __global__ void eval_tc_reduce_kernel(const double* __restrict__ part, int nblocks, double* __restrict__ out) {
     // 32 groups x 8 statistics: group g sums CTAs g, g+32, ... ; the 32 group sums fold in a fixed order
     __shared__ double sh[32][8];
@@ -224,6 +218,7 @@ __global__ void eval_tc_reduce_kernel(const double* __restrict__ part, int nbloc
     }
 }
 
+// Tensor-core variant of osb_actor_eval (O <= 512; layer 1 K-chunked above 64); same arguments and outputs.
 int osb_actor_eval_tc(const float* theta_actor, int O, int A, const float* obs, const float* act,
                       const float* logp, const float* adv_r, const float* adv_c, const float* mu_old,
                       const float* logstd_old, const float* moments, const float* lagrange,

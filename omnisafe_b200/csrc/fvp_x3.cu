@@ -231,7 +231,6 @@ using namespace osb;
 
 extern "C" {
 
-int osb_tc_grid_blocks(long long rows, int net_mask);
 int osb_x3_fvp_backward(const float* theta_actor, const float* vec, int O, int A, const float* obs, long long total, int stride,
                         const float* dmu, float* gpart, float* stats_scratch, void* stream);
 

@@ -11,8 +11,10 @@
 //   conjugate_gradients                  utils/math.py:L86-132
 #include "common.cuh"
 #include "mlp.cuh"
+#include "optim.cuh"
 #include <cooperative_groups.h>
 #include <string.h>
+#include <type_traits>
 
 namespace osb {
 
@@ -108,28 +110,32 @@ __global__ void __launch_bounds__(OT) clip_adam_kernel(AdamArgs p) {
     if (p.do_clip && p.max_grad_norm > 0.f) {
         float tot = 0.f;
         for (int b = 0; b < p.NB; ++b) tot += p.sumsq_part[net * p.NB + b];
-        const float coef = fminf(p.max_grad_norm / (sqrtf(tot) + 1e-6f), 1.0f);
-        g *= coef;
+        g *= clip_coef(p.max_grad_norm, tot);
         p.grad[q] = g;
     }
     if (!p.do_adam) return;
     g *= p.grad_scale;
-    // torch.optim.Adam, single-tensor path (betas 0.9/0.999, eps 1e-8, no weight decay)
-    const int t = p.adam_step[net];
-    const double bc1 = 1.0 - pow(0.9, (double)t);
-    const double bc2 = 1.0 - pow(0.999, (double)t);
-    const float step_size = (float)((double)p.lr[net] / bc1);
-    const float bc2_sqrt = (float)sqrt(bc2);
+    const AdamBias b = adam_bias(p.lr[net], p.adam_step[net]);
     float m = p.m[q], v = p.v[q];
-    m = __fadd_rn(m, __fmul_rn(0.1f, __fadd_rn(g, -m)));                       // exp_avg.lerp_(grad, 1-b1)
-    v = __fadd_rn(__fmul_rn(v, 0.999f), __fmul_rn(__fmul_rn(0.001f, g), g));   // mul_(b2).addcmul_(g, g, 1-b2)
-    const float denom = __fadd_rn(__fdiv_rn(sqrtf(v), bc2_sqrt), 1e-8f);
-    p.theta[q] = __fadd_rn(p.theta[q], __fmul_rn(-step_size, __fdiv_rn(m, denom)));
+    p.theta[q] = adam_update(g, p.theta[q], m, v, b);
     p.m[q] = m; p.v[q] = v;
 }
 
-// Single-rank fast path: partial reduction + critic L2 term + per-network clip + Adam in ONE
-// cooperative launch (grid.sync() between the norm reduction and the parameter update).
+// Multi-rank all-reduce of the fused kernel: a one-shot exchange over NVLink peer memory (cudaIpc-mapped buffers,
+// NVSwitch gives every peer full bandwidth).  Each rank publishes its clipped flat gradient (99 KB) in its own exchange
+// buffer, raises a step flag in every peer's memory, waits for the peers' flags, then sums the peers' buffers in rank
+// order (deterministic, identical on every rank) straight into the Adam update -- the reference's order
+// clip -> average -> step (policy_gradient.py:L437-443; distributed.py:L193-198 avg_grads).
+struct P2PExchange {
+    float* const* peer_buf;        // [world] exchange buffers, each [2][P] (double-buffered by step parity)
+    unsigned int* const* peer_flag; // [world] flag arrays, each [2][world]
+    int world, rank;
+    unsigned int step_id;          // monotonically increasing, identical on all ranks
+    int* error_flag;               // set when a peer does not show up (timeout) instead of hanging the GPU
+};
+
+// Partial reduction + critic L2 term + per-network clip (+ all-reduce) + Adam in ONE cooperative launch
+// (grid.sync() between the norm reduction and the parameter update).
 struct FusedOptArgs {
     ReduceArgs r;
     float* m;
@@ -137,6 +143,10 @@ struct FusedOptArgs {
     float max_grad_norm;
     float lr[3];
 };
+struct P2POptArgs : FusedOptArgs {
+    P2PExchange x;
+};
+template <bool P2P> using OptArgs = std::conditional_t<P2P, P2POptArgs, FusedOptArgs>;
 
 // Fixed-order sum of the per-CTA partial gradients of one parameter, 16 loads in flight at a time
 // (the in-order issue would otherwise serialise one L2 round trip per small batch).
@@ -155,7 +165,7 @@ __device__ __forceinline__ float reduce_partials16(const float* __restrict__ gpa
 // After the grid barrier: warp 0 of every CTA folds the per-CTA squared norms (lanes stride over CTAs, fixed
 // butterfly) into the clip scale and the Adam step sizes; in CTA 0 warp 1 folds the loss statistics.
 __device__ __forceinline__ void clip_scale_and_stats(const FusedOptArgs& p, int net, int step_t, float* s_scale,
-                                                     float* s_step, float* s_bc2) {
+                                                     AdamBias* s_bias) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int G = gridDim.x;
     if (warp == 0 || (warp == 1 && blockIdx.x == 0)) {
@@ -164,10 +174,8 @@ __device__ __forceinline__ void clip_scale_and_stats(const FusedOptArgs& p, int 
         tot = warp_sum(tot); t2 = warp_sum(t2);
         if (warp == 0) {
             if (lane == 0) {
-                *s_scale = (p.max_grad_norm > 0.f) ? fminf(p.max_grad_norm / (sqrtf(tot) + 1e-6f), 1.0f) : 1.0f;
-                const double bc1 = 1.0 - pow(0.9, (double)step_t), bc2 = 1.0 - pow(0.999, (double)step_t);
-                *s_step = (float)((double)p.lr[net] / bc1);
-                *s_bc2 = (float)sqrt(bc2);
+                *s_scale = clip_coef(p.max_grad_norm, tot);
+                *s_bias = adam_bias(p.lr[net], step_t);
             }
         } else {
             float acc[4] = {0.f, 0.f, 0.f, 0.f};
@@ -178,24 +186,31 @@ __device__ __forceinline__ void clip_scale_and_stats(const FusedOptArgs& p, int 
             for (int i = 0; i < 4; ++i) acc[i] = warp_sum(acc[i]);
             if (lane == 0) {
                 p.r.adam_step[net] = step_t;                   // every CTA read it before the grid barrier
-                const float inv = acc[3] > 0.f ? 1.f / acc[3] : 0.f;
-                float* ts = p.r.train_stats + net * 8;
-                ts[0] += acc[0] * inv + ((net != 0) ? p.r.critic_norm_coef * t2 : 0.f);
-                ts[1] += acc[1] * inv;
-                ts[2] += acc[2] * inv;
-                ts[3] += 1.f;
+                fold_train_stats(p.r.train_stats + net * 8, acc, net != 0, p.r.critic_norm_coef, &t2);
             }
         }
     }
 }
 
-__global__ void __launch_bounds__(OT) optim_fused_kernel(FusedOptArgs p) {
+__device__ __forceinline__ unsigned int ld_acquire_sys(const unsigned int* p) {
+    unsigned int v;
+    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
+    return v;
+}
+__device__ __forceinline__ void st_release_sys(unsigned int* p, unsigned int v) {
+    asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
+}
+
+// P2P = false: one rank.  P2P = true: several ranks, averaged through the P2PExchange between clip and Adam.
+template <bool P2P>
+__global__ void __launch_bounds__(OT) optim_fused_kernel(OptArgs<P2P> p) {
     namespace cg = cooperative_groups;
-    if (p.r.stop_flag && *p.r.stop_flag) return;          // uniform across the grid
+    if (p.r.stop_flag && *p.r.stop_flag) return;          // uniform across the grid and across ranks
     const int net = blockIdx.y;
     const bool active = ((p.r.net_mask >> net) & 1) != 0;
     __shared__ float red[OT / 32], red2[OT / 32];
-    __shared__ float s_scale, s_step, s_bc2;
+    __shared__ float s_scale;
+    __shared__ AdamBias s_bias;
     const NetLayout L = net_layout(net, p.r.O, p.r.A);
     const int noff = net_offset(net, p.r.O, p.r.A);
     const int pl = blockIdx.x * OT + threadIdx.x;
@@ -220,114 +235,50 @@ __global__ void __launch_bounds__(OT) optim_fused_kernel(FusedOptArgs p) {
         }
     }
     cg::this_grid().sync();
-    if (active) clip_scale_and_stats(p, net, step_t, &s_scale, &s_step, &s_bc2);
+    if (active) clip_scale_and_stats(p, net, step_t, &s_scale, &s_bias);
     __syncthreads();
-    if (active && pl < L.size) {
-        g *= s_scale;
-        p.r.grad[q] = g;
-        float m = p.m[q], v = p.v[q];
-        m = __fadd_rn(m, __fmul_rn(0.1f, __fadd_rn(g, -m)));
-        v = __fadd_rn(__fmul_rn(v, 0.999f), __fmul_rn(__fmul_rn(0.001f, g), g));
-        const float denom = __fadd_rn(__fdiv_rn(sqrtf(v), s_bc2), 1e-8f);
-        p.r.theta[q] = __fadd_rn(th, __fmul_rn(-s_step, __fdiv_rn(m, denom)));
-        p.m[q] = m; p.v[q] = v;
-    }
-}
-
-// Multi-rank fast path: partial reduction + clip + ALL-REDUCE + Adam in ONE cooperative kernel.  The
-// all-reduce is a one-shot exchange over NVLink peer memory (cudaIpc-mapped buffers, NVSwitch gives every
-// peer full bandwidth): each rank publishes its clipped flat gradient (99 KB) in its own exchange buffer,
-// raises a step flag in every peer's memory, waits for the peers' flags, then sums the peers' buffers in
-// rank order (deterministic, identical on every rank) straight into the Adam update -- the reference's
-// order clip -> average -> step (policy_gradient.py:L437-443; distributed.py:L193-198 avg_grads).
-struct P2POptArgs {
-    FusedOptArgs f;
-    float* const* peer_buf;        // [world] exchange buffers, each [2][P] (double-buffered by step parity)
-    unsigned int* const* peer_flag; // [world] flag arrays, each [2][world]
-    int world, rank;
-    unsigned int step_id;          // monotonically increasing, identical on all ranks
-    int* error_flag;               // set when a peer does not show up (timeout) instead of hanging the GPU
-};
-
-__device__ __forceinline__ unsigned int ld_acquire_sys(const unsigned int* p) {
-    unsigned int v;
-    asm volatile("ld.acquire.sys.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_release_sys(unsigned int* p, unsigned int v) {
-    asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
-__global__ void __launch_bounds__(OT) optim_fused_p2p_kernel(P2POptArgs a) {
-    namespace cg = cooperative_groups;
-    const FusedOptArgs& p = a.f;
-    if (p.r.stop_flag && *p.r.stop_flag) return;          // uniform across the grid and across ranks
-    const int net = blockIdx.y;
-    const bool active = ((p.r.net_mask >> net) & 1) != 0;
-    __shared__ float red[OT / 32], red2[OT / 32];
-    __shared__ float s_scale, s_step, s_bc2;
-    const NetLayout L = net_layout(net, p.r.O, p.r.A);
-    const int noff = net_offset(net, p.r.O, p.r.A);
-    const int pl = blockIdx.x * OT + threadIdx.x;
-    const int q = noff + pl;
-    const int par = (int)(a.step_id & 1u);
-    float g = 0.f, th = 0.f;
-    int step_t = 0;
-    if (active) {
-        step_t = p.r.adam_step[net] + 1;
-        if (pl < L.size) {
-            g = reduce_partials16(p.r.gpart, p.r.nblocks, p.r.P, q);
-            th = p.r.theta[q];
-            if (net != 0 && p.r.critic_norm_coef > 0.f) g += 2.f * p.r.critic_norm_coef * th;
-        }
-        float s = warp_sum(g * g), s2 = warp_sum(net != 0 ? th * th : 0.f);
-        if ((threadIdx.x & 31) == 0) { red[threadIdx.x >> 5] = s; red2[threadIdx.x >> 5] = s2; }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            float t = 0.f, t2 = 0.f;
-            for (int w = 0; w < OT / 32; ++w) { t += red[w]; t2 += red2[w]; }
-            p.r.sumsq_part[net * gridDim.x + blockIdx.x] = t;
-            p.r.sumsq_part[(3 + net) * gridDim.x + blockIdx.x] = t2;
-        }
-    }
-    cg::this_grid().sync();
-    if (active) clip_scale_and_stats(p, net, step_t, &s_scale, &s_step, &s_bc2);
-    __syncthreads();
-    // ---- publish the clipped gradient, exchange flags over NVLink, sum the peers ---------------------
-    float* mine = a.peer_buf[a.rank] + (size_t)par * p.r.P;
-    if (pl < L.size) mine[q] = active ? g * s_scale : 0.f;
-    __threadfence_system();
-    cg::this_grid().sync();
-    if (blockIdx.x == 0 && blockIdx.y == 0) {
-        if ((int)threadIdx.x < a.world)       // tell every peer (and myself) that my buffer for this step is ready
-            st_release_sys(a.peer_flag[threadIdx.x] + par * a.world + a.rank, a.step_id);
-        if ((int)threadIdx.x < a.world) {     // wait until every peer's buffer for this step is ready
-            const unsigned int* f = a.peer_flag[a.rank] + par * a.world + threadIdx.x;
-            const long long t0 = clock64();
-            while (ld_acquire_sys(f) != a.step_id) {
-                if (clock64() - t0 > 4000000000LL) { *a.error_flag = 1; break; }   // ~2 s: fail instead of hanging
+    bool exchange_ok = true;
+    if constexpr (P2P) {
+        // ---- publish the clipped gradient, exchange flags over NVLink ---------------------------------------
+        const P2PExchange& x = p.x;
+        const int par = (int)(x.step_id & 1u);
+        float* mine = x.peer_buf[x.rank] + (size_t)par * p.r.P;
+        if (pl < L.size) mine[q] = active ? g * s_scale : 0.f;
+        __threadfence_system();
+        cg::this_grid().sync();
+        if (blockIdx.x == 0 && blockIdx.y == 0) {
+            if ((int)threadIdx.x < x.world)       // tell every peer (and myself) that my buffer for this step is ready
+                st_release_sys(x.peer_flag[threadIdx.x] + par * x.world + x.rank, x.step_id);
+            if ((int)threadIdx.x < x.world) {     // wait until every peer's buffer for this step is ready
+                const unsigned int* f = x.peer_flag[x.rank] + par * x.world + threadIdx.x;
+                const long long t0 = clock64();
+                while (ld_acquire_sys(f) != x.step_id) {
+                    if (clock64() - t0 > 4000000000LL) { *x.error_flag = 1; break; }   // ~2 s: fail instead of hanging
+                }
             }
         }
+        cg::this_grid().sync();
+        // a peer that never published (time-out above) leaves its buffer stale: skip the step instead of applying garbage --
+        // the sticky error flag is raised by the host (distributed.p2p_check), the parameters stay those of the last good step
+        exchange_ok = *((volatile int*)x.error_flag) == 0;
     }
-    cg::this_grid().sync();
-    // a peer that never published (time-out above) leaves its buffer stale: skip the step instead of applying garbage --
-    // the sticky error flag is raised by the host (distributed.p2p_check), the parameters stay those of the last good step
-    const bool exchange_ok = *((volatile int*)a.error_flag) == 0;
     if (active && pl < L.size && exchange_ok) {
-        float sum = 0.f;
-        for (int r = 0; r < a.world; ++r) {
-            const float* pb = a.peer_buf[r] + (size_t)par * p.r.P;
-            float v;
-            asm volatile("ld.relaxed.sys.global.f32 %0, [%1];" : "=f"(v) : "l"(pb + q) : "memory");
-            sum += v;
+        if constexpr (P2P) {                     // sum the peers in rank order
+            const int par = (int)(p.x.step_id & 1u);
+            float sum = 0.f;
+            for (int r = 0; r < p.x.world; ++r) {
+                const float* pb = p.x.peer_buf[r] + (size_t)par * p.r.P;
+                float v;
+                asm volatile("ld.relaxed.sys.global.f32 %0, [%1];" : "=f"(v) : "l"(pb + q) : "memory");
+                sum += v;
+            }
+            g = sum / (float)p.x.world;
+        } else {
+            g *= s_scale;
         }
-        const float gavg = sum / (float)a.world;
-        p.r.grad[q] = gavg;
+        p.r.grad[q] = g;
         float m = p.m[q], v = p.v[q];
-        m = __fadd_rn(m, __fmul_rn(0.1f, __fadd_rn(gavg, -m)));
-        v = __fadd_rn(__fmul_rn(v, 0.999f), __fmul_rn(__fmul_rn(0.001f, gavg), gavg));
-        const float denom = __fadd_rn(__fdiv_rn(sqrtf(v), s_bc2), 1e-8f);
-        p.r.theta[q] = __fadd_rn(th, __fmul_rn(-s_step, __fdiv_rn(m, denom)));
+        p.r.theta[q] = adam_update(g, th, m, v, s_bias);
         p.m[q] = m; p.v[q] = v;
     }
 }
@@ -344,11 +295,7 @@ __global__ void lagrange_update_kernel(const double* __restrict__ window_sums, f
     const float g = (float)(-(jc - (double)cost_limit));
     float lam = state[0], m = state[1], v = state[2];
     const int t = (int)state[3] + 1;
-    const double bc1 = 1.0 - pow(0.9, (double)t), bc2 = 1.0 - pow(0.999, (double)t);
-    m = __fadd_rn(m, __fmul_rn(0.1f, __fadd_rn(g, -m)));
-    v = __fadd_rn(__fmul_rn(v, 0.999f), __fmul_rn(__fmul_rn(0.001f, g), g));
-    const float denom = __fadd_rn(__fdiv_rn(sqrtf(v), (float)sqrt(bc2)), 1e-8f);
-    lam = __fadd_rn(lam, __fmul_rn(-(float)((double)lambda_lr / bc1), __fdiv_rn(m, denom)));
+    lam = adam_update(g, lam, m, v, adam_bias(lambda_lr, t));
     lam = fmaxf(lam, 0.f);
     if (upper_bound >= 0.f) lam = fminf(lam, upper_bound);
     state[0] = lam; state[1] = m; state[2] = v; state[3] = (float)t;
@@ -482,6 +429,33 @@ __global__ void axpy_kernel(const float* __restrict__ x, const float* __restrict
 
 using namespace osb;
 
+// Arguments of the partial reduction, shared by grad_reduce_kernel and optim_fused_kernel
+static ReduceArgs reduce_args(const float* gpart, const float* stats_part, int nblocks, int O, int A, const float* theta,
+                              float* grad, float critic_norm_coef, int net_mask, float* sumsq_part, int* adam_step,
+                              float* train_stats, const int* stop_flag) {
+    return {gpart, stats_part, nblocks, actor_layout(O, A).size + 2 * critic_layout(O, A).size, O, A,
+            const_cast<float*>(theta), grad, critic_norm_coef, net_mask, sumsq_part, adam_step, train_stats, stop_flag};
+}
+
+// osb_optim_fused (x == NULL) and osb_optim_fused_p2p (x = the peer-memory exchange between the ranks)
+static int optim_fused(const float* gpart, const float* stats_part, int nblocks, int O, int A, float* theta, float* grad,
+                       float* adam_m, float* adam_v, int* adam_step, float critic_norm_coef, float max_grad_norm,
+                       float lr_actor, float lr_critic_r, float lr_critic_c, int net_mask, float* sumsq_part,
+                       float* train_stats, const int* stop_flag, const P2PExchange* x, void* stream) {
+    OSB_CHECK_ARG(gpart && stats_part && theta && grad && adam_m && adam_v && adam_step && sumsq_part && train_stats, "null pointer");
+    OSB_CHECK_ARG(!x || (x->peer_buf && x->peer_flag && x->error_flag && x->world > 1 && x->world <= OT && x->rank >= 0 &&
+                         x->rank < x->world), "bad p2p argument");
+    P2POptArgs a = {{reduce_args(gpart, stats_part, nblocks, O, A, theta, grad, critic_norm_coef, net_mask, sumsq_part,
+                                 adam_step, train_stats, stop_flag),
+                     adam_m, adam_v, max_grad_norm, {lr_actor, lr_critic_r, lr_critic_c}},
+                    x ? *x : P2PExchange{}};
+    void* args[] = {x ? (void*)&a : (void*)static_cast<FusedOptArgs*>(&a)};   // one rank: the base part only
+    osb_count_launch();
+    OSB_CUDA(cudaLaunchCooperativeKernel(x ? (void*)optim_fused_kernel<true> : (void*)optim_fused_kernel<false>,
+                                         dim3(osb_optim_blocks(O, A), 3), dim3(OT), args, 0, (cudaStream_t)stream));
+    return OSB_OK;
+}
+
 extern "C" {
 
 int osb_optim_blocks(int O, int A) {
@@ -497,11 +471,8 @@ int osb_grad_reduce(const float* gpart, const float* stats_part, int nblocks, in
                     float* sumsq_part, int* adam_step, float* train_stats, const int* stop_flag,
                     void* stream) {
     OSB_CHECK_ARG(gpart && stats_part && theta && grad && sumsq_part && adam_step && train_stats, "null pointer");
-    ReduceArgs p;
-    p.gpart = gpart; p.stats_part = stats_part; p.nblocks = nblocks; p.O = O; p.A = A;
-    p.P = actor_layout(O, A).size + 2 * critic_layout(O, A).size;
-    p.theta = const_cast<float*>(theta); p.grad = grad; p.critic_norm_coef = critic_norm_coef; p.net_mask = net_mask;
-    p.sumsq_part = sumsq_part; p.adam_step = adam_step; p.train_stats = train_stats; p.stop_flag = stop_flag;
+    const ReduceArgs p = reduce_args(gpart, stats_part, nblocks, O, A, theta, grad, critic_norm_coef, net_mask, sumsq_part,
+                                     adam_step, train_stats, stop_flag);
     grad_reduce_kernel<<<dim3(osb_optim_blocks(O, A), 3), OT, 0, (cudaStream_t)stream>>>(p);
     OSB_LAUNCH_CHECK();
     return OSB_OK;
@@ -534,19 +505,9 @@ int osb_optim_fused(const float* gpart, const float* stats_part, int nblocks, in
                     float critic_norm_coef, float max_grad_norm, float lr_actor, float lr_critic_r,
                     float lr_critic_c, int net_mask, float* sumsq_part, float* train_stats,
                     const int* stop_flag, void* stream) {
-    OSB_CHECK_ARG(gpart && stats_part && theta && grad && adam_m && adam_v && adam_step && sumsq_part && train_stats, "null pointer");
-    FusedOptArgs p;
-    p.r.gpart = gpart; p.r.stats_part = stats_part; p.r.nblocks = nblocks; p.r.O = O; p.r.A = A;
-    p.r.P = actor_layout(O, A).size + 2 * critic_layout(O, A).size;
-    p.r.theta = theta; p.r.grad = grad; p.r.critic_norm_coef = critic_norm_coef; p.r.net_mask = net_mask;
-    p.r.sumsq_part = sumsq_part; p.r.adam_step = adam_step; p.r.train_stats = train_stats; p.r.stop_flag = stop_flag;
-    p.m = adam_m; p.v = adam_v; p.max_grad_norm = max_grad_norm;
-    p.lr[0] = lr_actor; p.lr[1] = lr_critic_r; p.lr[2] = lr_critic_c;
-    void* args[] = {&p};
-    osb_count_launch();
-    OSB_CUDA(cudaLaunchCooperativeKernel((void*)optim_fused_kernel, dim3(osb_optim_blocks(O, A), 3), dim3(OT), args, 0,
-                                         (cudaStream_t)stream));
-    return OSB_OK;
+    return optim_fused(gpart, stats_part, nblocks, O, A, theta, grad, adam_m, adam_v, adam_step, critic_norm_coef,
+                       max_grad_norm, lr_actor, lr_critic_r, lr_critic_c, net_mask, sumsq_part, train_stats, stop_flag,
+                       nullptr, stream);
 }
 
 // ---- NVLink peer-memory exchange buffers (cudaIpc) -----------------------------------------------------
@@ -581,23 +542,10 @@ int osb_optim_fused_p2p(const float* gpart, const float* stats_part, int nblocks
                         float lr_critic_r, float lr_critic_c, int net_mask, float* sumsq_part,
                         float* train_stats, const int* stop_flag, void* peer_buf, void* peer_flag,
                         int world, int rank, unsigned step_id, int* error_flag, void* stream) {
-    OSB_CHECK_ARG(gpart && stats_part && theta && grad && adam_m && adam_v && adam_step && sumsq_part && train_stats, "null pointer");
-    OSB_CHECK_ARG(peer_buf && peer_flag && error_flag && world > 1 && world <= OT && rank >= 0 && rank < world, "bad p2p argument");
-    P2POptArgs a;
-    FusedOptArgs& p = a.f;
-    p.r.gpart = gpart; p.r.stats_part = stats_part; p.r.nblocks = nblocks; p.r.O = O; p.r.A = A;
-    p.r.P = actor_layout(O, A).size + 2 * critic_layout(O, A).size;
-    p.r.theta = theta; p.r.grad = grad; p.r.critic_norm_coef = critic_norm_coef; p.r.net_mask = net_mask;
-    p.r.sumsq_part = sumsq_part; p.r.adam_step = adam_step; p.r.train_stats = train_stats; p.r.stop_flag = stop_flag;
-    p.m = adam_m; p.v = adam_v; p.max_grad_norm = max_grad_norm;
-    p.lr[0] = lr_actor; p.lr[1] = lr_critic_r; p.lr[2] = lr_critic_c;
-    a.peer_buf = (float* const*)peer_buf; a.peer_flag = (unsigned int* const*)peer_flag;
-    a.world = world; a.rank = rank; a.step_id = step_id; a.error_flag = error_flag;
-    void* args[] = {&a};
-    osb_count_launch();
-    OSB_CUDA(cudaLaunchCooperativeKernel((void*)optim_fused_p2p_kernel, dim3(osb_optim_blocks(O, A), 3), dim3(OT), args, 0,
-                                         (cudaStream_t)stream));
-    return OSB_OK;
+    const P2PExchange x = {(float* const*)peer_buf, (unsigned int* const*)peer_flag, world, rank, step_id, error_flag};
+    return optim_fused(gpart, stats_part, nblocks, O, A, theta, grad, adam_m, adam_v, adam_step, critic_norm_coef,
+                       max_grad_norm, lr_actor, lr_critic_r, lr_critic_c, net_mask, sumsq_part, train_stats, stop_flag,
+                       &x, stream);
 }
 
 int osb_lagrange_update(const double* window_sums, float cost_limit, float lambda_lr,

@@ -1283,9 +1283,6 @@ static size_t rollout_smem_bytes(int O) {   // O = network input width
 
 extern "C" {
 
-int osb_episode_window(const unsigned char* flags, const float* epfin, int T, int N, int W,
-                       float* ring, int* meta, double* window_sums, void* stream);
-
 // Opaque-struct-free C ABI: the caller passes plain device pointers.
 int osb_env_reset(int O, int A, int max_episode_steps, unsigned seed, unsigned term_threshold,
                   unsigned env_id_offset, float cost_threshold, int obs_normalize, int N,

@@ -1074,8 +1074,6 @@ static int launch_grad_tc(const TcArgs& p, int nblocks, cudaStream_t stream) {
 
 extern "C" {
 
-int osb_update_grid_blocks(int mb_count);
-
 // CTAs along x of the tensor-core kernel: three networks share the 148 SMs (49 each); a single
 // network (full-batch actor passes of the natural-gradient family) spreads over all of them.
 int osb_tc_grid_blocks(long long rows, int net_mask) {

@@ -33,6 +33,7 @@
 // forward-only statistics pass), supplied dOUT (Fisher-vector product backward).
 #include "common.cuh"
 #include "mlp.cuh"
+#include "optim.cuh"
 #include "x3.cuh"
 
 namespace osb {
@@ -500,10 +501,9 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
             const float inv_b = 1.0f / (float)count;
             const bool have_tiles = (int)blockIdx.x < ntiles;
             if (FUSED && tid == NEPI - 1) {        // Adam bias corrections of this minibatch's step, off the critical path
-                const int step_t = step_t0 + mb + 1;
-                const double bc1 = 1.0 - pow(0.9, (double)step_t), bc2 = 1.0 - pow(0.999, (double)step_t);
-                sScal[8] = (float)((double)p.lr[net] / bc1);
-                sScal[9] = (float)sqrt(bc2);
+                const AdamBias b = adam_bias(p.lr[net], step_t0 + mb + 1);
+                sScal[8] = b.step_size;
+                sScal[9] = b.bc2_sqrt;
             }
 #pragma unroll 1
             for (int tile = blockIdx.x; tile < ntiles; tile += G, ++it) {
@@ -949,11 +949,7 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
             if (own) { pre_th = __ldcg(p.theta_rw + noff + p0 + tid); pre_m = __ldcg(p.adam_m + noff + p0 + tid); pre_v = __ldcg(p.adam_v + noff + p0 + tid); }
             // torch-Adam step of one parameter (+ its three bf16 pieces in the weight-tile image)
             auto adam_store = [&](int qg, float g, float th, float m, float v, bool img) {
-                const float step_size = sScal[8], bc2_sqrt = sScal[9];
-                m = __fadd_rn(m, __fmul_rn(0.1f, __fadd_rn(g, -m)));                       // exp_avg.lerp_(grad, 1 - beta1)
-                v = __fadd_rn(__fmul_rn(v, 0.999f), __fmul_rn(__fmul_rn(0.001f, g), g));   // mul_(beta2).addcmul_(g, g, 1 - beta2)
-                const float denom = __fadd_rn(__fdiv_rn(sqrtf(v), bc2_sqrt), 1e-8f);
-                const float th_new = __fadd_rn(th, __fmul_rn(-step_size, __fdiv_rn(m, denom)));
+                const float th_new = adam_update(g, th, m, v, {sScal[8], sScal[9]});
                 __stcg(p.theta_rw + qg, th_new);
                 __stcg(p.adam_m + qg, m); __stcg(p.adam_v + qg, v);
                 if (img && img_off >= 0) {           // where the weight tiles expect them
@@ -978,7 +974,7 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                 for (int b = lane; b < G; b += 32) { tot += __ldcg(p.sumsq_part + (net * 2 + 0) * G + b); t2 += __ldcg(p.sumsq_part + (net * 2 + 1) * G + b); }
                 tot = warp_sum(tot); t2 = warp_sum(t2);
                 if (lane == 0) {
-                    sScal[0] = (p.max_grad_norm > 0.f) ? fminf(p.max_grad_norm / (sqrtf(tot) + 1e-6f), 1.0f) : 1.0f;
+                    sScal[0] = clip_coef(p.max_grad_norm, tot);
                     sScal[3] = t2;
                 }
             } else if (warp == 1 && blockIdx.x == 0) {               // loss statistics of this minibatch (logger means)
@@ -991,14 +987,8 @@ __global__ void __launch_bounds__(NTX3, 1) minibatch_grad_x3_kernel(X3Args p) {
                 if (lane == 0) { sScal[4] = acc[0]; sScal[5] = acc[1]; sScal[6] = acc[2]; sScal[7] = acc[3]; }
             }
             epi_bar_sync();
-            if (blockIdx.x == 0 && tid == 0) {
-                const float inv = sScal[7] > 0.f ? 1.f / sScal[7] : 0.f;
-                float* ts = p.train_stats + net * 8;
-                ts[0] += sScal[4] * inv + ((net != 0) ? p.critic_norm_coef * sScal[3] : 0.f);
-                ts[1] += sScal[5] * inv;
-                ts[2] += sScal[6] * inv;
-                ts[3] += 1.f;
-            }
+            if (blockIdx.x == 0 && tid == 0)
+                fold_train_stats(p.train_stats + net * 8, sScal + 4, net != 0, p.critic_norm_coef, sScal + 3);
             const float clipc = sScal[0];
             const unsigned int xstep = p.step_base + (unsigned int)mb;
             const int xpar = (int)(xstep & 1u);
@@ -1106,8 +1096,6 @@ __global__ void x3_mask_mean_kernel(const float* __restrict__ stats_part, int nb
 using namespace osb;
 
 extern "C" {
-
-int osb_tc_grid_blocks(long long rows, int net_mask);
 
 static long long* g_x3_dbg = nullptr;
 // development aid: clock64 stamps of CTA (0, 0) of the next launches go to buf (2048 long long), NULL turns it off

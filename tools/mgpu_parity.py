@@ -4,7 +4,7 @@ through every data-parallel path of the library --
 
   bf16x3 persistent kernel, clipped slices pushed over NVLink peer memory inside the kernel   (the bench path)
   bf16x3 per-minibatch kernels + reduce / clip / ncclAllReduce / Adam as separate launches      (OSB_X3_NO_FUSE, OSB_NO_P2P)
-  fp32 tiles + optim_fused_p2p_kernel (one-shot peer-memory all-reduce inside the optimiser kernel)
+  fp32 tiles + optim_fused_kernel<true> (one-shot peer-memory all-reduce inside the optimiser kernel)
   fp32 tiles + NCCL
 
 -- and must land on the reference's parameters (fp32 bar) with bit-identical parameters on all ranks.
